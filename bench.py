@@ -40,6 +40,25 @@ WORKLOADS = {
 }
 
 
+DUMP_LIMIT = 64_000_000                                    # --dump-outputs: bytes of all files together (.npy headers included)
+DUMP_COUNTERS = ("n_ext", "n_miss", "n_emissive_hits", "n_shadow", "n_cont", "n_unoccluded")   # rows of frame_counters.npy
+
+
+def dump_arrays(rad, counters):
+    """The --dump-outputs files of a frame: radiance (h x w x 4 float32) and the per-bounce counters (float64).  When they
+    would not fit DUMP_LIMIT, the radiance becomes a fixed, seeded sample of pixels (float32 RGBA) plus those pixels' indices
+    (float64, exact): 24 bytes per sampled pixel, the sample sized so that every file fits with room for the .npy headers."""
+    out = {"frame_counters": counters}
+    if rad.nbytes + counters.nbytes + 4096 <= DUMP_LIMIT:
+        out["radiance"] = rad
+        return out
+    flat = rad.reshape(-1, 4)
+    n = (DUMP_LIMIT - counters.nbytes - 4096) // 24
+    pix = np.sort(np.random.default_rng(0).choice(len(flat), n, replace=False))
+    out["radiance_sample"], out["radiance_sample_pixels"] = flat[pix], pix.astype(np.float64)
+    return out
+
+
 def load_workload_scene(name, w, h, copies=183):
     """Scene arrays + camera of a workload.  Synthetic10M is generated (raytracing_b200/synthetic.py) and its BVH
     is built on the host by every rank (deterministic, so all ranks hold identical bytes)."""
@@ -307,7 +326,14 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="RT_OPT_OVERLAP=0: shadow pass on the render stream (no concurrency with the next traversal)")
     ap.add_argument("--no-smem-bvh", action="store_true", help="RT_OPT_SMEM_BVH=0: fetch BVH records through L1 even for small scenes")
     ap.add_argument("--copies", type=int, default=183, help="Synthetic10M: number of ShaderBalls copies (183 = 10 026 570 triangles)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (radiance, per-bounce ray counters) to DIR/<name>.npy, "
+                         "at most 64 MB in all; DIR is created if missing and is best kept outside the source tree")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference does not run it")
     workload = WORKLOADS[args.scene]
     if args.impl == "reference":
         run_reference_arm(args, workload)
@@ -429,6 +455,8 @@ def main():
         ms_per_step = float(ms_total[0]) / steps
         launches = ctx.launch_count() - launches0
         sampler.join(timeout=2)
+        if args.dump_outputs and workload == WORKLOADS[args.scene]:
+            dump_outputs(args.dump_outputs, ctx, mb, slab.device)
         # Per-kernel durations for the roofline.  In the timed region above the frame is ONE CUDA-graph launch and the shadow
         # pass of a bounce runs inside the next bounce's traversal kernel, so per-launch CUDA events are neither possible (graph)
         # nor would they separate the two passes: the same K steps are run once more, in this same process, with
@@ -478,6 +506,21 @@ def main():
                      "per-phase kernels: [closest-hit trace(b) + shadow pass(b-1)] -> hit/miss queues -> shade(b), one CUDA graph per frame"))
 
         return types.SimpleNamespace(**{k: v for k, v in locals().items() if k not in ("workload",)})
+
+    def dump_outputs(out_dir, ctx, mb, device):
+        """What a caller of the timed path receives after its last step: the accumulated radiance (h x w x 4, rows of every
+        rank) and the frame's per-bounce ray counters, written by rank 0 (dump_arrays)."""
+        rad = torch.from_numpy(ctx.read_radiance()).to(device)          # other ranks' rows are zero here
+        st = ctx.frame_stats()
+        counters = torch.tensor(np.stack([st[k][: mb + 1].astype(np.float64) for k in DUMP_COUNTERS]), device=device)
+        if world > 1:
+            dist.reduce(rad, dst=0)
+            dist.reduce(counters, dst=0)
+        if rank != 0:
+            return
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in dump_arrays(rad.cpu().numpy(), counters.cpu().numpy()).items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
 
     def destroy_context(c):
         """Rank 0's context owns the fused-gather buffer that the other ranks have mapped through CUDA IPC: they unmap (destroy

@@ -106,6 +106,12 @@ static const int* PaddedRankingTile()
     return padded.data();
 }
 
+// Tables that replace the compiled-in ones (ref_set_sampler_tables); empty: the reference's own tables.
+static std::vector<int> g_sobol, g_scrambling, g_ranking;
+static const void* SobolTable() { return g_sobol.empty() ? (const void*)sobol_256spp_256d : (const void*)g_sobol.data(); }
+static const void* ScramblingTable() { return g_scrambling.empty() ? (const void*)scramblingTile : (const void*)g_scrambling.data(); }
+static const void* RankingTable() { return g_ranking.empty() ? (const void*)PaddedRankingTile() : (const void*)g_ranking.data(); }
+
 class RefCpuIntegrator : public Integrator
 {
 public:
@@ -203,7 +209,7 @@ protected:
         fn(N(), rays_[in].p, ray_counter_[in].p, pixel_indices_[in].p, hits_.p, scene_.triangles.data(),
             scene_.lights.data(), scene_.emissive.data(), scene_.materials.data(), scene_.textures.data(),
             scene_.texture_data.data(), bounce, width_, height_, sample_counter_.p, &scene_.info,
-            (void*)sobol_256spp_256d, (void*)scramblingTile, (void*)PaddedRankingTile(),
+            (void*)SobolTable(), (void*)ScramblingTable(), (void*)RankingTable(),
             throughputs_.p, rays_[out].p, ray_counter_[out].p, pixel_indices_[out].p,
             shadow_rays_.p, shadow_ray_counter_.p, shadow_pixel_indices_.p, direct_light_samples_.p, radiance_.p);
         if (bounce < (std::uint32_t)kMaxStatBounces)
@@ -358,6 +364,18 @@ void ref_enable_white_furnace(void* handle, int e) { ((RefHandle*)handle)->integ
 void ref_sampler_tables(const int** sobol, const int** scrambling, const int** ranking)
 {
     *sobol = (const int*)sobol_256spp_256d; *scrambling = (const int*)scramblingTile; *ranking = (const int*)rankingTile;
+}
+// Other tables of the same sizes for the blue-noise kernels (the ranking table gets the same 256 zeros of padding as the
+// compiled-in one); null pointers restore the compiled-in tables.
+void ref_set_sampler_tables(const int* sobol, const int* scrambling, const int* ranking)
+{
+    if (!sobol || !scrambling || !ranking) { g_sobol.clear(); g_scrambling.clear(); g_ranking.clear(); return; }
+    const size_t n_sobol = sizeof(sobol_256spp_256d) / sizeof(int), n_scrambling = sizeof(scramblingTile) / sizeof(int),
+                 n_ranking = sizeof(rankingTile) / sizeof(rankingTile[0]);
+    g_sobol.assign(sobol, sobol + n_sobol);
+    g_scrambling.assign(scrambling, scrambling + n_scrambling);
+    g_ranking.assign(ranking, ranking + n_ranking);
+    g_ranking.resize(n_ranking + 256, 0);
 }
 void ref_set_sampler(void* handle, int blue_noise) { ((RefHandle*)handle)->integrator->SetSamplerType(blue_noise ? Integrator::SamplerType::kBlueNoise : Integrator::SamplerType::kRandom); }
 void ref_enable_denoiser(void* handle, int e) { ((RefHandle*)handle)->integrator->EnableDenoiser(e != 0); }

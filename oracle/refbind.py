@@ -24,6 +24,18 @@ def available(libm: bool = False) -> bool:
 
 from raytracing_b200.camera import default_camera  # noqa: E402,F401
 
+def set_sampler_tables(tables, libm: bool = False):
+    """Process-wide: the blue-noise kernels of libref[_libm].so read copies of these (sobol, scrambling, ranking) tables of the
+    reference's sizes from now on; None restores the tables the reference compiled in."""
+    L = C.CDLL(os.path.join(REF_DIR, "libref_libm.so" if libm else "libref.so"))
+    L.ref_set_sampler_tables.argtypes = [C.c_void_p] * 3
+    if tables is None:
+        L.ref_set_sampler_tables(None, None, None)
+        return
+    t = [np.ascontiguousarray(x, dtype=np.int32) for x in tables]
+    assert [len(x) for x in t] == [65536, 131072, 131072]
+    L.ref_set_sampler_tables(*[x.ctypes.data_as(C.c_void_p) for x in t])
+
 
 class RefRenderer:
     """One reference scene + integrator instance on the CPU."""

@@ -1,5 +1,6 @@
 """Shared helpers for the parity tests."""
 import glob
+import hashlib
 import os
 
 import numpy as np
@@ -41,20 +42,22 @@ def bits(a):
     return u
 
 
+def digest(*arrays):
+    """SHA-256 (first 128 bits, in hex) over arrays: float arrays as their bit patterns (see bits), others as stored.  Stands in for a stored
+    output in the bit-exact comparisons with the reference (tests/golden/ref)."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.asarray(a)
+        h.update(bits(a).tobytes() if a.dtype.kind == "f" else np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()[:32]
+
+
 def synthetic_sampler_tables(seed=20260923):
     """Seeded stand-ins for the blue-noise sampler's tables (same shapes and value ranges as the reference's
     utils/blue_noise_sampler.hpp, which is reference data and not committed here): any tables exercise the same lookups."""
     rng = np.random.default_rng(seed)
     return (rng.integers(0, 256, 65536, dtype=np.int32), rng.integers(0, 256, 131072, dtype=np.int32),
             rng.integers(0, 256, 131072, dtype=np.int32))
-
-
-def reference_sampler_tables():
-    """The reference's own tables, read out of oracle/_ref/libref.so when that library was built; else None."""
-    from oracle import refbind
-    if not refbind.available():
-        return None
-    return refbind.RefRenderer().sampler_tables()
 
 
 def fuzz_configs(n=12, seed=77):

@@ -10,11 +10,17 @@ import pytest
 from oracle.orcbind import Oracle
 from raytracing_b200 import hostapi, scene_io
 from raytracing_b200.camera import default_camera
-from tests.helpers import bits, scene, synthetic_sampler_tables
+from tests.helpers import bits, digest, scene, synthetic_sampler_tables
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PROC_OBJ = os.path.join(REPO, "tests", "golden", "scenes", "procedural.obj")
-REF_ASSETS = "/root/reference/assets"
+REF_GOLDEN = os.path.join(REPO, "tests", "golden", "ref")          # what the reference made of the inputs below (make_ref_fixtures.py)
+
+
+def reference_record(key):
+    import json
+    with open(os.path.join(REF_GOLDEN, "expected.json")) as f:
+        return json.load(f)[key]
 
 
 def write_hdr(path, rgbe, rle=True):
@@ -285,32 +291,29 @@ def test_hdr_reader_cases_load_like_the_reference(tmp_path):
         assert hdr_cases.digest(*_load_env(str(tmp_path / "e.hdr"))) == expected[name], name
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="the reference's own pipeline only exists in the build container")
+GENERATED_OBJ = [("tex", "quads"), ("quads", "polys", "tex", "neg", "groups")]     # features of the even / odd seeds
+
+
 @pytest.mark.parametrize("seed", range(8))
 def test_generated_obj_renders_like_the_reference_pipeline(tmp_path, seed):
     """A generated textured OBJ (quads, polygons, random materials, PNG / TGA maps) through BOTH whole pipelines on the CPU: the
-    reference's Scene + Bvh + kernels (oracle/_ref) against host loader + host BVH + oracle — primary hits and every radiance
-    bit.  (560 further seeds were run once with 0 differences.)"""
-    from oracle import refbind
+    reference's Scene + Bvh + kernels (oracle/_ref, stored as digests) against host loader + host BVH + oracle — primary hits
+    and every radiance bit.  (560 further seeds were run once with 0 differences.)"""
     from tests import obj_cases
-    if not refbind.available():
-        pytest.skip("oracle/_ref/libref.so not built")
-    features = ("quads", "polys", "tex", "neg", "groups") if seed % 2 else ("tex", "quads")
-    obj = obj_cases.write_case(str(tmp_path), obj_cases.random_scene(200 + seed, features))
+    obj = obj_cases.write_case(str(tmp_path), obj_cases.random_scene(200 + seed, GENERATED_OBJ[seed % 2]))
     w, h, mb = 96, 54, 5
     cam = hostapi.default_camera(w, h); cam["position"][:3] = (0.2, -3.4, 0.4)
-    r = refbind.RefRenderer().open_obj("/root/reference", obj)
-    r.begin(w, h); r.set_camera(cam); r.set_max_bounces(mb); r.integrate()
     s = hostapi.HostScene(obj)
     s.add_directional_light((-0.6, -1.5, 3.5), (15, 10, 5)); s.build_bvh()
-    s.finalize(env_path=os.path.join(REF_ASSETS, "ibl", "CGSkies_0036_free.hdr"))
+    env, env_w, env_h = scene_io.load_env()                     # the reference's decoding of its environment map
+    s.finalize(env=env, env_width=env_w, env_height=env_h)
     a = s.arrays(); s.close()
     acc, hits, st = Oracle(a).render(cam, w, h, mb)
+    ref = reference_record("generated_obj/%d" % seed)
     assert (hits["primitive_id"] != 0xFFFFFFFF).sum() > 100
-    assert np.array_equal(hits["primitive_id"], r.primary_hits()["primitive_id"])
-    assert np.array_equal(st["n_ext"][: mb + 1], r.stats()["n_ext"][: mb + 1])
-    assert np.array_equal(bits(acc[..., :3]), bits(r.radiance()[..., :3]))
-    r.close()
+    assert digest(hits["primitive_id"]) == ref["primitive_id"]
+    assert st["n_ext"][: mb + 1].tolist() == ref["n_ext"]
+    assert digest(acc[..., :3]) == ref["radiance"]
 
 
 def test_bvh_builder_on_generated_soups(tmp_path):
@@ -342,23 +345,12 @@ def test_bvh_builder_on_generated_soups(tmp_path):
             os.environ.pop(k, None) if v is None else os.environ.__setitem__(k, v)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="the reference's own loader only exists in the build container")
-def test_obj_reader_matches_the_reference_loader_live(tmp_path):
-    """Fresh generated scenes (other seeds than the committed expectations) and 120 000 numbers in ten notations through the
-    reference's own loader (oracle/_ref) and through host/obj_reader.cpp."""
-    from oracle import refbind
-    from tests import obj_cases
-    if not refbind.available():
-        pytest.skip("oracle/_ref/libref.so not built")
+LIVE_OBJ_CASES = [(seed, features) for seed in range(100, 112)
+                  for features in (("quads", "polys"), ("quads", "polys", "neg", "groups", "tabs", "crlf", "vcolor", "badmtl", "smooth"))]
 
-    def reference_arrays(obj):
-        return refbind.RefRenderer().open_obj("/root/reference", obj).scene()
-    k = 0
-    for seed in range(100, 112):
-        for features in (("quads", "polys"), ("quads", "polys", "neg", "groups", "tabs", "crlf", "vcolor", "badmtl", "smooth")):
-            obj = obj_cases.write_case(str(tmp_path / ("r%d" % k)), obj_cases.random_scene(seed, features))
-            assert _same_scene_arrays(_scene_arrays_from_obj(obj), reference_arrays(obj)) is None, (seed, features)
-            k += 1
+
+def numbers_obj():
+    """120 000 numbers in ten notations as vertex coordinates."""
     rng = np.random.default_rng(9)
     vals = np.concatenate([rng.uniform(-3, 3, 60000), rng.normal(0, 100, 30000), 10.0 ** rng.uniform(-6, 4, 30000)])
     rng.shuffle(vals)
@@ -366,16 +358,25 @@ def test_obj_reader_matches_the_reference_loader_live(tmp_path):
     toks = [notations[i % len(notations)] % v for i, v in enumerate(vals)]
     lines = ["mtllib s.mtl", "vn 0 0 1", "usemtl a"] + ["v %s %s %s" % tuple(toks[3 * i: 3 * i + 3]) for i in range(len(toks) // 3)]
     lines += ["f %d//1 %d//1 %d//1" % (i + 1, i + 2, i + 3) for i in range(0, len(toks) // 3 - 2, 3)]
-    obj = obj_cases.write_case(str(tmp_path / "numbers"), {"s.obj": "\n".join(lines) + "\n", "s.mtl": "newmtl a\nKd 0.5 0.5 0.5\n"})
-    assert _same_scene_arrays(_scene_arrays_from_obj(obj), reference_arrays(obj)) is None
+    return {"s.obj": "\n".join(lines) + "\n", "s.mtl": "newmtl a\nKd 0.5 0.5 0.5\n"}
+
+
+def test_obj_reader_matches_the_reference_loader_live(tmp_path):
+    """Generated scenes (other seeds than tests/golden/obj) and 120 000 numbers in ten notations through host/obj_reader.cpp,
+    against digests of what the reference's own loader (oracle/_ref) made of the same files."""
+    from tests import hdr_cases, obj_cases
+    from tests.ref_cases import scene_arrays_digest
+    ref = reference_record("obj_reader_live")
+    for k, (seed, features) in enumerate(LIVE_OBJ_CASES):
+        obj = obj_cases.write_case(str(tmp_path / ("r%d" % k)), obj_cases.random_scene(seed, features))
+        assert scene_arrays_digest(_scene_arrays_from_obj(obj)) == ref["%d_%s" % (seed, "_".join(features))], (seed, features)
+    obj = obj_cases.write_case(str(tmp_path / "numbers"), numbers_obj())
+    assert scene_arrays_digest(_scene_arrays_from_obj(obj)) == ref["numbers"]
     # environment maps, another seed than the committed digests
-    from tests import hdr_cases
-    from tests.golden.make_obj_fixtures import reference_env
-    for i, (name, data) in enumerate(hdr_cases.cases(seed=31).items()):
+    for name, data in hdr_cases.cases(seed=31).items():
         with open(tmp_path / "e.hdr", "wb") as f:
             f.write(data)
-        root = tmp_path / ("env%d" % i); root.mkdir()
-        assert hdr_cases.digest(*_load_env(str(tmp_path / "e.hdr"))) == hdr_cases.digest(*reference_env(str(root), data)), name
+        assert hdr_cases.digest(*_load_env(str(tmp_path / "e.hdr"))) == ref["env/" + name], name
 
 
 TEXTURE_DIR = os.path.join(REPO, "tests", "golden", "textures")
@@ -427,14 +428,10 @@ def test_texture_files_decode_like_the_reference(tmp_path):
         assert np.array_equal(_pack_like_stb(im.convert("RGB") if im.mode == "P" else im), expected[n + ":texels"]), n
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="the reference's own loader only exists in the build container")
-def test_image_textures_match_the_reference_loader(tmp_path):
-    """The same textured OBJ through the reference's own Scene (tinyobj + LoadSTB, compiled into oracle/_ref) and through
-    host/image_loader.cpp: Texture[] records, texel words and packed material words identical (scene.cpp:155-186,276-300)."""
+def textured_obj_images(directory):
+    """PNG (RGB, RGBA, grey, grey+alpha, palette with and without tRNS, 16 bit, 1 bit) and TGA (RGB, RLE RGBA, grey) files
+    written into `directory`; returns their names."""
     from PIL import Image
-    from oracle import refbind
-    if not refbind.available():
-        pytest.skip("oracle/_ref/libref.so not built")
     rng = np.random.default_rng(21)
 
     def rnd(shape, dtype=np.uint8, hi=256):
@@ -455,40 +452,50 @@ def test_image_textures_match_the_reference_loader(tmp_path):
     imgs["grey16.png"] = Image.fromarray(rnd((5, 9), np.uint16, 65536))
     imgs["bits1.png"] = Image.fromarray(rnd((11, 19), hi=2) * 255, "L").convert("1")
     for name, im in imgs.items():
+        path = os.path.join(str(directory), name)
         if name == "rgba_rle.tga":
-            im.save(str(tmp_path / name), compression="tga_rle")
+            im.save(path, compression="tga_rle")
         elif name == "pal_trns.png":
-            im.save(str(tmp_path / name), transparency=bytes([0, 128, 255, 7]))
+            im.save(path, transparency=bytes([0, 128, 255, 7]))
         else:
-            im.save(str(tmp_path / name))
-    obj = _textured_obj(tmp_path, list(imgs))
-    g = refbind.RefRenderer().open_obj("/root/reference", obj).scene()        # absolute OBJ path; the CWD only serves Finalize()
+            im.save(path)
+    return list(imgs)
+
+
+def test_image_textures_match_the_reference_loader(tmp_path):
+    """The same textured OBJ through host/image_loader.cpp and, stored as digests, through the reference's own Scene (tinyobj +
+    LoadSTB, compiled into oracle/_ref): Texture[] records, texel words and packed material words identical
+    (scene.cpp:155-186,276-300); then freshly generated JPEG / Adam7 files and the reference's assets/checker3.jpg."""
+    ref = reference_record("image_textures")
+    obj = _textured_obj(tmp_path, textured_obj_images(tmp_path))
     s = hostapi.HostScene(obj)
     s.add_directional_light((-0.6, -1.5, 3.5), (15, 10, 5))
     s.build_bvh()
-    s.finalize(env_path=os.path.join(REF_ASSETS, "ibl", "CGSkies_0036_free.hdr"))
+    s.finalize(env=np.zeros(4, dtype=np.float32), env_width=1, env_height=1)
     a = s.arrays()
-    assert len(g["textures"]) == len(imgs)
+    assert len(a["textures"]) == ref["textures"]
     for f in ("width", "height", "data_start"):                   # the record's padding word is uninitialised in the reference
-        assert np.array_equal(a["textures"][f], g["textures"][f]), f
-    assert np.array_equal(a["texels"], g["texels"])
-    assert a["materials"].tobytes() == g["materials"].tobytes()
-    assert np.array_equal(a["triangles"]["mtlIndex"], g["triangles"]["mtlIndex"])
+        assert digest(a["textures"][f]) == ref[f], f
+    assert digest(a["texels"]) == ref["texels"]
+    assert digest(a["materials"]) == ref["materials"]
+    assert digest(a["triangles"]["mtlIndex"]) == ref["mtlIndex"]
     for v in ("v1", "v2", "v3"):
-        assert np.array_equal(bits(a["triangles"][v]["texcoord"][:, :2]), bits(g["triangles"][v]["texcoord"][:, :2]))
+        assert digest(a["triangles"][v]["texcoord"][:, :2]) == ref[v + ".texcoord"], v
     s.close()
-    # freshly generated JPEG / Adam7 files (another seed than the committed fixtures) and the JPEG the reference ships
-    import shutil
+    # freshly generated JPEG / Adam7 files (another seed than the committed fixtures)
     from tests.golden import make_texture_fixtures as mk
     fresh = tmp_path / "fresh"
     names = mk.make_files(str(fresh), np.random.default_rng(77))
-    shutil.copy(os.path.join(REF_ASSETS, "checker3.jpg"), fresh / "checker3.jpg")
-    names.append("checker3.jpg")
-    ref = mk.reference_texels(str(fresh), names)
+    assert sorted(names) == sorted(ref["fresh"])
     work = tmp_path / "work"; work.mkdir()
     got = _load_texture_files(str(fresh), names, work)
     for n in names:
-        assert got[n][:2] == ref[n][:2] and np.array_equal(got[n][2], ref[n][2]), n
+        w, h, texels = got[n]
+        assert [w, h, digest(texels)] == ref["fresh"][n], n
+    # the JPEG the reference ships with its assets
+    work = tmp_path / "assets"; work.mkdir()
+    for n, (w, h, texels) in _load_texture_files(REF_GOLDEN, sorted(ref["assets"]), work).items():
+        assert [w, h, digest(texels)] == ref["assets"][n], n
 
 
 @pytest.mark.gpu
@@ -519,28 +526,24 @@ def test_textured_obj_renders_like_the_oracle(tmp_path):
     r.close(); s.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="reference assets only exist in the build container")
 @pytest.mark.parametrize("name", ["CornellBox", "ShaderBalls", "CornellBox_Dragon"])
-def test_loader_and_builder_reproduce_reference_dumps(name):
-    """Same OBJ/MTL/HDR in -> the arrays the reference's own Scene + Bvh::BuildCPU + LoadHDR produced (fixtures)."""
-    s = hostapi.HostScene(os.path.join(REF_ASSETS, name + ".obj"))
+def test_loader_and_builder_reproduce_reference_dumps(tmp_path, name):
+    """Same OBJ/MTL/HDR in -> the arrays the reference's own Scene + Bvh::BuildCPU + LoadHDR produced (stored per field as
+    digests).  CornellBox is the reference's whole OBJ; of the two large ones, runs of 64 consecutive faces, one in every 128, with
+    the lines they use are kept (tests/ref_cases.py: obj_face_subset).  The environment map is read from every 50th scanline of the reference's file and
+    compared with those rows of its decoding."""
+    from tests.ref_cases import ENV_ROW_STEP, loader_digests, write_env_rows, write_loader_input
+    s = hostapi.HostScene(write_loader_input(name, tmp_path))
     s.add_directional_light((-0.6, -1.5, 3.5), (15, 10, 5))      # main.cpp:58
     s.build_bvh()
-    s.finalize(env_path=os.path.join(REF_ASSETS, "ibl", "CGSkies_0036_free.hdr"))
-    a, g = s.arrays(), scene(name)
-    assert len(a["triangles"]) == len(g["triangles"]) and len(a["nodes"]) == len(g["nodes"])
-    for v in ("v1", "v2", "v3"):
-        for f in ("position", "texcoord", "normal"):
-            assert np.array_equal(bits(a["triangles"][v][f][:, :3]), bits(g["triangles"][v][f][:, :3])), (v, f)
-    assert np.array_equal(a["triangles"]["mtlIndex"], g["triangles"]["mtlIndex"])
-    for k in ("bounds_min", "bounds_max"):
-        assert np.array_equal(bits(a["nodes"][k][:, :3]), bits(g["nodes"][k][:, :3]))
-    for k in ("offset", "num_primitives_axis"):
-        assert np.array_equal(a["nodes"][k], g["nodes"][k])
-    assert a["materials"].tobytes() == g["materials"].tobytes()
-    assert np.array_equal(bits(a["lights"]["origin"][:, :3]), bits(g["lights"]["origin"][:, :3]))
-    assert np.array_equal(a["emissive"], g["emissive"]) and a["scene_info"].tobytes() == g["scene_info"].tobytes()
-    assert np.array_equal(bits(a["env"]), bits(g["env"]))
+    s.finalize(env_path=write_env_rows(tmp_path))
+    a = s.arrays()
+    got, ref = loader_digests(a), reference_record("loader/" + name)
+    assert [k for k in ref if got[k] != ref[k]] == [], (got["counts"], ref["counts"])
+    env, env_w, env_h = scene_io.load_env()
+    rows = env.reshape(env_h, env_w, 4)[::ENV_ROW_STEP]
+    assert (int(a["env_width"]), int(a["env_height"])) == (rows.shape[1], rows.shape[0])
+    assert np.array_equal(bits(a["env"]), bits(rows.reshape(-1)))
     s.close()
 
 
